@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — throughput of the Predict()/Perceive() hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--streams S] [--step-bytes B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--streams S] [--step-bytes B] [--dump-outputs DIR]
     python bench.py --impl reference ...           # the reference's own CPU implementation on the box's host cores
 
 Workload = BASELINE.json configs[1]: synthetic enwik8-shaped ASCII text (tools/gen_synth.py, seed 0xE9E80001),
@@ -18,6 +18,8 @@ every stream by --step-bytes bytes (8x as many coded bits). One stream = one ref
             stream, against MEASURED_PEAKS.json; `kernels` lists every bulk kernel's measured time per coded bit so that
             the share of each (and the pole) is visible.
 `bpc`       cross entropy of the coded prefix from the device's probabilities, next to the reference's on the same bytes.
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) so that two builds can be compared output for
+output: the inputs depend only on the arguments.
 Multi-GPU (torchrun): independent files per rank, no data-path collective (weak scaling); time = max over ranks.
 """
 import argparse
@@ -103,6 +105,20 @@ def bench_stream(n_file, stream_id=0):
 
 N_E2E = 10
 N_AGG = 3
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(directory, arrays, limit=DUMP_LIMIT):
+    """Write every array as directory/<name>.npy (float32 or float64). Past `limit` bytes in all, each array is replaced by the
+    same fixed, seeded sample of its flattened elements (sorted positions), sized so that the files stay within the limit."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        if total > limit:
+            keep = a.size * limit // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def file_bytes(B, W, K):
@@ -152,7 +168,11 @@ def main():
     ap.add_argument("--aggregate-streams", type=int, default=int(os.environ.get("CMIXB200_BENCH_AGG", "7")), help="files per GPU for the aggregate figure (0 = skip)")
     ap.add_argument("--step-bytes", type=int, default=1024)
     ap.add_argument("--cpu-sample-bytes", type=int, default=4096)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the probabilities the last timed step returned to DIR/p.npy "
+                    "(float32, one row of step-bytes x 8 per stream; with several ranks DIR/p_rank<r>.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -273,6 +293,9 @@ def main():
     sampler.stop_flag = True
     sampler.join(timeout=2)
     value = total_bytes / dt / 1e6
+    if args.dump_outputs:
+        last = torch.stack([st["d_out"][(st["pos"] - B) * 8:st["pos"] * 8] for st in head]).cpu().numpy()
+        dump_outputs(args.dump_outputs, {"p" if world == 1 else "p_rank%d" % rank: last}, DUMP_LIMIT // world)
 
     # ---- end to end through the C-ABI with pinned HOST buffers: the same streams continue ----
     preds = [st["P"] for st in head]

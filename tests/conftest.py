@@ -1,3 +1,4 @@
+import lzma
 import os
 import subprocess
 import sys
@@ -43,6 +44,15 @@ def golden(request):
 @pytest.fixture(scope="session")
 def golden_text():
     return Golden("text208")
+
+
+@pytest.fixture(scope="session")
+def english_dic(tmp_path_factory):
+    """The reference's WRT dictionary (`cmix -c english.dic`), stored xz-compressed by tools/make_ref_golden.py."""
+    path = tmp_path_factory.mktemp("dic") / "english.dic"
+    with lzma.open(os.path.join(ROOT, "tests", "golden", "english.dic.xz")) as f:
+        path.write_bytes(f.read())
+    return str(path)
 
 
 @pytest.fixture(scope="session")

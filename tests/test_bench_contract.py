@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -29,3 +30,20 @@ def test_other_ranks_of_the_reference_arm_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"], capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_dump_outputs_samples_past_the_limit(tmp_path):
+    """bench.dump_outputs (--dump-outputs): arrays within the limit are written whole; past it every array becomes the same
+    seeded sample of its elements on every run, and the files stay within the limit."""
+    code = ("import sys, numpy as np; sys.path.insert(0, %r); import bench\n"
+            "a = np.arange(1000, dtype=np.float32).reshape(10, 100)\n"
+            "bench.dump_outputs(sys.argv[1], {'p': a})\n"
+            "for d in sys.argv[2:]: bench.dump_outputs(d, {'p': a, 'q': a.astype(np.float64)}, limit=3000)\n" % ROOT)
+    dirs = [str(tmp_path / d) for d in ("whole", "s1", "s2")]
+    subprocess.run([sys.executable, "-c", code] + dirs, check=True, cwd=ROOT)
+    np.testing.assert_array_equal(np.load(os.path.join(dirs[0], "p.npy")), np.arange(1000, dtype=np.float32).reshape(10, 100))
+    p1, q1 = np.load(os.path.join(dirs[1], "p.npy")), np.load(os.path.join(dirs[1], "q.npy"))
+    assert p1.dtype == np.float32 and q1.dtype == np.float64 and p1.nbytes + q1.nbytes <= 3000 and p1.size == 250
+    assert np.all(np.diff(p1) > 0)
+    np.testing.assert_array_equal(p1, np.load(os.path.join(dirs[2], "p.npy")))
+    np.testing.assert_array_equal(q1, np.load(os.path.join(dirs[2], "q.npy")))

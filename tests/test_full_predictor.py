@@ -14,8 +14,6 @@ import pytest
 
 from conftest import ROOT
 
-DICT = os.path.join(ROOT, "oracle", "_ref", "english.dic")
-
 
 def _load(name):
     z = np.load(os.path.join(ROOT, "tests", "golden", name + ".npz"))
@@ -43,12 +41,13 @@ def test_paq8_host_build_matches_reference_codes(paq8_check, tmp_path, name):
     assert np.array_equal(got, g["crc_p8"][:got.size]) and got.size == n * 8 // 4096
 
 
-def test_paq8_tables_are_the_reference_tables(tmp_path):
-    """The hex tables in paq8_host.h against the reference's own initialisers (build container only)."""
-    if not os.path.exists("/root/reference/src/models/paq8.cpp"):
-        pytest.skip("reference sources not present on this box")
-    r = subprocess.run(["python", os.path.join(ROOT, "tools", "make_paq8_tables.py"), "--check"], capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout + r.stderr
+def test_paq8_tables_are_the_reference_tables():
+    """The hex tables in paq8_host.h against what the reference's own initialisers produce (tools/make_ref_golden.py)."""
+    from make_paq8_tables import differences
+    z = np.load(os.path.join(ROOT, "tests", "golden", "ref_tables.npz"))
+    want = {k[len("paq8_"):]: z[k].tobytes().hex() for k in z.files if k.startswith("paq8_")}
+    assert len(want) == 15
+    assert differences(want) == []
 
 
 # ------------------------------------------------------------------------------------------------ GPU
@@ -103,13 +102,12 @@ def test_everything_resident_equals_the_reference(cm, name):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not os.path.exists(DICT), reason="oracle/_ref/english.dic not staged")
-def test_everything_resident_with_dictionary_and_pretraining(cm):
+def test_everything_resident_with_dictionary_and_pretraining(cm, english_dic):
     """cmix -c english.dic in out: WRT code words in the stream, Pretrain() over header + dictionary before the first bit."""
     g = _load("full_wrt")
-    d = open(DICT, "rb").read()
+    d = open(english_dic, "rb").read()
     pre = bytes([0, (len(d) >> 24) & 255, (len(d) >> 16) & 255, (len(d) >> 8) & 255, len(d) & 255]) + d.replace(b"\n", b" ")
-    p, crc_fx, crc_p8, first = _run_resident(cm, g, dictionary=DICT, pretrain=pre, n=2048)
+    p, crc_fx, crc_p8, first = _run_resident(cm, g, dictionary=english_dic, pretrain=pre, n=2048)
     _assert_matches(g, p, crc_fx, crc_p8, first)
 
 

@@ -13,7 +13,6 @@ import pytest
 
 from conftest import ROOT, Golden
 
-DICT = os.path.join(ROOT, "oracle", "_ref", "english.dic")
 FIXTURES = ["fxcm_text", "fxcm_bin", "fxcm_wrt"]
 
 
@@ -31,16 +30,14 @@ def fxcm_check(tmp_path_factory):
 
 
 @pytest.mark.parametrize("name", FIXTURES)
-def test_host_build_matches_reference_codes(fxcm_check, tmp_path, name):
+def test_host_build_matches_reference_codes(fxcm_check, english_dic, tmp_path, name):
     g = _load(name)
     use_dict = bool(g["dictionary"][0])
-    if use_dict and not os.path.exists(DICT):
-        pytest.skip("oracle/_ref/english.dic not staged (make -C oracle ref)")
     prefix = str(tmp_path / "d")
     g["stream"].tofile(prefix + ".stream")
     g["lstmfx"].tofile(prefix + ".lstmfx.u32")
     crc_out = prefix + ".crc"
-    r = subprocess.run([fxcm_check, prefix, DICT if use_dict else "-", str(g["stream"].size), crc_out], capture_output=True, text=True)
+    r = subprocess.run([fxcm_check, prefix, english_dic if use_dict else "-", str(g["stream"].size), crc_out], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
     got = np.fromfile(crc_out, dtype=np.uint32)
     bad = np.nonzero(got != g["crc"])[0]
@@ -48,16 +45,13 @@ def test_host_build_matches_reference_codes(fxcm_check, tmp_path, name):
 
 
 def test_tables_are_the_reference_tables():
-    """The byte-class tables are spelled as digit strings in fxcm_host.h; when the reference is present compare them."""
+    """The byte-class tables are spelled as digit strings in fxcm_host.h; compare them with the reference's (tools/make_ref_golden.py)."""
     import re
-    ref_path = "/root/reference/src/models/fxcmv1.cpp"
-    if not os.path.exists(ref_path):
-        pytest.skip("reference sources not present on this box")
-    ref = open(ref_path).read()
+    ref = np.load(os.path.join(ROOT, "tests", "golden", "ref_tables.npz"))
     mine = open(os.path.join(ROOT, "cmix_b200", "csrc", "fxcm_host.h")).read()
     for theirs, ours in (("wrt_2b", "wrt2"), ("wrt_3b", "wrt3"), ("wrt_4b", "wrt4")):
-        body = re.sub(r"//.*", "", re.search(theirs + r"\[\d+\]\s*=\s*\{(.*?)\};", ref, re.S).group(1))
-        want = [int(x) for x in re.findall(r"\d+", body)]
+        want = ref["fxcm_" + theirs].tolist()
+        assert len(want) == 256
         m = re.search(r"fill_digits\(T\." + ours + r", 256,(.*?)\);", mine, re.S)
         got = [int(c, 16) for c in "".join(re.findall(r'"(.*?)"', m.group(1))).replace(" ", "")]
         assert got == want, theirs
@@ -102,15 +96,14 @@ def test_device_fxcm_chain_matches_reference_codes(cm, name):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not os.path.exists(DICT), reason="oracle/_ref/english.dic not staged")
-def test_device_fxcm_with_dictionary_and_pretraining(cm):
+def test_device_fxcm_with_dictionary_and_pretraining(cm, english_dic):
     """cmix -c english.dic: WRT code words in the stream, Pretrain() over header + dictionary before the first bit."""
     g = _load("fxcm_wrt")
-    d = open(DICT, "rb").read()
+    d = open(english_dic, "rb").read()
     pre = bytes([0, (len(d) >> 24) & 255, (len(d) >> 16) & 255, (len(d) >> 8) & 255, len(d) & 255]) + d.replace(b"\n", b" ")
     n = 2048                                                   # 3 CRC blocks... keep the GPU test short: pretraining dominates
     g = dict(g); g["stream"] = g["stream"][:n]
-    got, first = _device_code_crcs(cm, g, dictionary=DICT, pretrain=pre)
+    got, first = _device_code_crcs(cm, g, dictionary=english_dic, pretrain=pre)
     assert np.array_equal(first, g["first_codes"])
     assert np.array_equal(got, g["crc"][:got.size])
 

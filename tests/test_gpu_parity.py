@@ -1,6 +1,6 @@
 """GPU parity tests (-m gpu): the CUDA path, called through the C-ABI, against
 (1) golden vectors dumped from the unmodified reference, (2) the oracle port on seeded
-inputs, (3) a fresh dump from oracle/_ref/oracle_dump when that binary travelled to the box.
+inputs, (3) the reference's probabilities over synthetic text, with every model group resident.
 Bit-exact everywhere (tolerance 0.0; north_star allows 1e-5 on probabilities)."""
 import os
 import subprocess
@@ -278,25 +278,20 @@ def test_device_coder_writes_the_reference_archive_bytes(cm, port, golden_text):
     assert np.array_equal(out, bits)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "oracle_dump")),
-                    reason="oracle/_ref/oracle_dump not shipped")
-def test_fresh_reference_dump_on_this_box(cm, tmp_path):
-    """Run the real reference here on 2 KB of synthetic enwik-shaped text and match it exactly,
-    then turn the probabilities into an archive and check the coder round trip and bpc."""
+def test_synthetic_text_equals_the_reference(cm):
+    """2 KB of synthetic enwik-shaped text through the complete resident predictor: every Predict() equals the reference's
+    (tools/make_ref_golden.py: oracle_dump over the same `cmix -n` stream), and so does the cross entropy."""
     from gen_synth import synth_text
-    from oracle_io import Dump, load_port
-    src = tmp_path / "in.txt"
-    src.write_bytes(synth_text(2000, 0xE9E80002))
-    subprocess.run([os.path.join(ROOT, "oracle", "_ref", "oracle_dump"), "dump", "n", str(src), str(tmp_path / "d"), "1"],
-                   check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    d = Dump(str(tmp_path / "d"))
-    P = cm.Predictor(d.vocab)
-    p = P.code_bytes(d.stream, d.ext, d.ppmd)
+    g = np.load(os.path.join(ROOT, "tests", "golden", "synth2k.npz"))
+    assert g["stream"][5:].tobytes() == synth_text(2000, 0xE9E80002)
+    P = cm.Predictor(g["vocab"])
+    p = P.code_bytes(g["stream"])
     P.close()
-    assert np.abs(p - d.p).max() <= TOL
-    bits = d.bits()
-    ideal = -np.log2(np.where(bits == 1, p, 1 - p).clip(1e-9, 1)).sum() / 8 / d.n_bytes * 8
-    ideal_ref = -np.log2(np.where(bits == 1, d.p, 1 - d.p).clip(1e-9, 1)).sum() / 8 / d.n_bytes * 8
+    assert np.abs(p - g["p"]).max() <= TOL
+    bits = np.unpackbits(g["stream"])
+    n_bytes = g["stream"].size
+    ideal = -np.log2(np.where(bits == 1, p, 1 - p).clip(1e-9, 1)).sum() / 8 / n_bytes * 8
+    ideal_ref = -np.log2(np.where(bits == 1, g["p"], 1 - g["p"]).clip(1e-9, 1)).sum() / 8 / n_bytes * 8
     assert abs(ideal - ideal_ref) <= 0.001          # bits per byte within 0.001 of the reference
 
 

@@ -4,9 +4,8 @@
     python tools/gen_synth.py binary 100000 out.bin [seed]
 
 text: enwik8/enwik9 shape. Words are drawn Zipf(s=1.07) over the ranks of the WRT dictionary
-(english.dic, rank = line number) when oracle/_ref/english.dic (a data file the oracle Makefile
-stages next to the reference binaries) is present, so that `cmix -c english.dic` finds dictionary
-hits; without it a seeded syllable lexicon of the same size class is used. Sentences of
+(english.dic, rank = line number; stored as tests/golden/english.dic.xz) so that `cmix -c english.dic`
+finds dictionary hits. Sentences of
 3+Poisson(14) words, 12 % capitalised starts, punctuation, [[wiki links]], entities, numbers,
 paragraphs, plus the wiki structures the text models key on (headings, lists, tables, templates,
 <math>/<nowiki>/<pre>, external links, bold/italic), every ~4 KB wrapped in a <page> element.
@@ -16,49 +15,24 @@ binary: alternating 64 KiB blocks of (i) x86-64 ELF-like code with repeating E8/
 targets and (ii) baseline-JPEG files whose scan is a real Huffman-coded stream (standard tables,
 random DCT coefficients, FF00 stuffing) so that a JPEG parser sees MCUs.
 """
+import lzma
 import os
 import sys
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-DICT_PATH = os.path.join(ROOT, "oracle", "_ref", "english.dic")
-
-_ONSETS = ["", "b", "c", "d", "f", "g", "h", "l", "m", "n", "p", "r", "s", "t", "w", "st", "tr", "ch", "sh", "th", "pr", "gr", "pl", "br"]
-_VOWELS = ["a", "e", "i", "o", "u", "ea", "ou", "io", "ai", "ee"]
-_CODAS = ["", "n", "r", "s", "t", "l", "m", "d", "ng", "nt", "st", "ck", "rd", "ll", "ss"]
-_COMMON = ("the of and to in a is that for it as was with be by on not he this are or his from at which but have an had they "
-           "you were their one all we can her has there been if more when will would who so no out up into than them only "
-           "its time some could these two may first then do any my now such like our over man even most made after also did "
-           "many before must through years where much your way well down should because each just those people how too little "
-           "state good very make world still own see men work long get here between both life being under never day same "
-           "another know while last might us great old year off come since against go came right used take three").split()
+DICT_PATH = os.path.join(ROOT, "tests", "golden", "english.dic.xz")
 
 
-def _lexicon(rng, n=6000):
-    words = list(_COMMON)
-    seen = set(words)
-    while len(words) < n:
-        k = 1 + min(3, int(rng.geometric(0.55)))
-        w = "".join(_ONSETS[rng.integers(len(_ONSETS))] + _VOWELS[rng.integers(len(_VOWELS))] + _CODAS[rng.integers(len(_CODAS))]
-                    for _ in range(k))
-        if w not in seen and 2 <= len(w) <= 14:
-            seen.add(w)
-            words.append(w)
-    return words
-
-
-def _words(rng):
-    if os.path.exists(DICT_PATH):
-        ws = [w for w in open(DICT_PATH, "rb").read().decode("latin-1").split("\n") if w and w.isascii() and w.isalpha()]
-        if len(ws) > 1000:
-            return ws
-    return _lexicon(rng)
+def _words():
+    with lzma.open(DICT_PATH) as f:
+        return [w for w in f.read().decode("latin-1").split("\n") if w and w.isascii() and w.isalpha()]
 
 
 class _TextGen:
     def __init__(self, seed):
         self.rng = np.random.default_rng(seed)
-        self.words = _words(self.rng)
+        self.words = _words()
         ranks = np.arange(1, len(self.words) + 1, dtype=np.float64)
         pz = ranks ** -1.07
         self.cdf = np.cumsum(pz / pz.sum())

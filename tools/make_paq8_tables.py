@@ -37,22 +37,29 @@ def tables():
     return dict(l.split() for l in (a + b).splitlines())
 
 
+def differences(t):
+    """Names of the tables whose hex strings in paq8_host.h differ from `t` (name -> hex)."""
+    src = open(os.path.join(ROOT, "cmix_b200", "csrc", "paq8_host.h")).read()
+    bad = []
+    for name, want in t.items():
+        field = {"state": r"&T\.state\[0\]\[0\]"}.get(name, r"T\." + name)
+        m = re.search(r"unhex\(" + field + r", \d+,(.*?)\);", src, re.S)
+        got = "".join(re.findall(r'"(.*?)"', m.group(1))) if m else ""
+        if got != want:
+            bad.append(name)
+    return bad
+
+
 def main():
     t = tables()
     if "--check" not in sys.argv:
         for k, v in t.items():
             print(k, v)
         return 0
-    src = open(os.path.join(ROOT, "cmix_b200", "csrc", "paq8_host.h")).read()
-    bad = 0
-    for name, want in t.items():
-        field = {"state": r"&T\.state\[0\]\[0\]"}.get(name, r"T\." + name)
-        m = re.search(r"unhex\(" + field + r", \d+,(.*?)\);", src, re.S)
-        got = "".join(re.findall(r'"(.*?)"', m.group(1))) if m else ""
-        if got != want:
-            print("table", name, "differs")
-            bad = 1
-    return bad
+    bad = differences(t)
+    for name in bad:
+        print("table", name, "differs")
+    return 1 if bad else 0
 
 
 if __name__ == "__main__":
